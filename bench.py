@@ -201,6 +201,20 @@ def measured_peaks():
     return {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0, "bf16_tflops_sustained": 1400.0}, "fallback"
 
 
+DUMP_BYTES = 64 * 2 ** 20
+
+
+def dump_outputs(outdir, outputs):
+    """What the timed path hands its caller -- the detection tensors [batch, ...] of one step -- as <outdir>/yolo_l<i>.npy
+    (float32).  Inputs and weights are seeded, so two builds can be compared file by file.  A batch larger than DUMP_BYTES
+    is cut to its leading images, the same ones on every run."""
+    os.makedirs(outdir, exist_ok=True)
+    per_image = sum(o[0].nbytes for o in outputs.values())
+    keep = max(1, DUMP_BYTES // per_image)
+    for i, o in outputs.items():
+        np.save(os.path.join(outdir, f"yolo_l{i}.npy"), np.ascontiguousarray(o[:keep], np.float32))
+
+
 def reference_run(args, workload):
     """`--impl reference`: the reference's own CPU implementation (oracle/_ref/libyolo2ref_fast.so = its sources
     compiled with the flags its Makefile recommends, AVX=1 OPENMP=1) on this box's host cores, batch 1 as its CLI
@@ -245,7 +259,12 @@ def main():
                     help="objectness threshold of the end-to-end detection path; 0 (default) = the lowest threshold >= 0.5 at which no\n"
                          "image yields more than 300 candidates: random-init heads sit at logit ~0, so the reference's demo default\n"
                          "0.24 would pass every one of the 22743 boxes of every image")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the detection tensors of the last one as DIR/<name>.npy (float32, "
+                         "at most 64 MB: a larger batch is cut to its leading images)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     if args.impl == "reference":
@@ -335,6 +354,8 @@ def main():
     ms_total = float(tmax.item())
     clocks = sampler.stop(t_wall0, t_wall1) if rank == 0 else None
     net.sync_outputs(quantized=bool(q), stream=stream)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, net.detection_outputs())
     sanity = {i: float(np.abs(o).mean()) for i, o in net.detection_outputs().items()}
     if not all(np.isfinite(v) and v > 0 for v in sanity.values()):
         raise SystemExit(f"bench.py: non-finite / empty detection outputs {sanity}")

@@ -1,11 +1,12 @@
 """INT8 input calibration (SURVEY 8f row 3): the host half -- histogram + KL search restated from
-entropy_calibration (yolov2_forward_network_quantized.c:1292-1398) -- must return the reference's multiplier bit for bit."""
+entropy_calibration (yolov2_forward_network_quantized.c:1292-1398) -- must return the reference's multiplier bit for bit
+(tests/golden/reference.json, "calibration")."""
 import numpy as np
 import pytest
 
 import ybtest_util as util
 
-pytestmark = pytest.mark.skipif(not util.have_ref(), reason="reference build absent")
+PARAMS = [(1.0 / 16, 4096), (1.0 / 4, 1024)]
 
 
 def _cases():
@@ -18,14 +19,13 @@ def _cases():
     yield "wide uniform", rng.random(400000) * 250.0
 
 
-@pytest.mark.parametrize("bin_width,max_bin", [(1.0 / 16, 4096), (1.0 / 4, 1024)])
+@pytest.mark.parametrize("bin_width,max_bin", PARAMS)
 def test_entropy_calibration_bit_identical_to_reference(bin_width, max_bin):
     import yolo2_light_b200 as yb
-    from oracle import ref
-    for name, arr in _cases():
+    expected = util.reference()["calibration"][f"{bin_width},{max_bin}"]
+    for (name, arr), theirs in zip(_cases(), expected, strict=True):
         a = np.asarray(arr, np.float32)
         mine = yb.api.entropy_calibration(a, bin_width, max_bin)
-        theirs = ref.entropy_calibration(a, bin_width, max_bin)
         assert np.float32(mine) == np.float32(theirs), (name, mine, theirs)
 
 

@@ -1,5 +1,6 @@
 """Generated model definitions == the reference's shipped assets, as seen by the reference's own parser; and the
-product parser == the reference parser on every generated model."""
+product parser == the reference parser on every generated model.  The assets and the reference parser's view of each
+model are stored in tests/golden/reference.json ("cfg_assets") and reference_arrays.npz ("parse_*")."""
 import os
 
 import numpy as np
@@ -8,7 +9,6 @@ import pytest
 import ybtest_util as util
 from yolo2_light_b200 import cfgs
 
-REF_BIN = "/root/reference/bin"
 ASSETS = [("yolov3", lambda: cfgs.yolov3(416, 416), "yolov3.cfg"), ("spp", cfgs.yolov3_spp, "yolov3-spp.cfg"),
           ("tiny", cfgs.yolov3_tiny, "yolov3-tiny.cfg"), ("xnor", cfgs.tiny_yolo_obj_xnor, "tiny-yolo-obj_xnor.cfg"),
           ("v2voc", cfgs.yolov2_voc, "yolov2-voc.cfg"), ("tinyvoc", cfgs.tiny_yolo_voc, "tiny-yolo-voc.cfg")]
@@ -23,13 +23,12 @@ TRAINING_KEYS = {"momentum", "decay", "angle", "saturation", "exposure", "hue", 
                  "bias_match"}
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_BIN), reason="reference tree absent")
 @pytest.mark.parametrize("name,build,asset", ASSETS)
 def test_generated_cfg_text_equals_reference_asset(name, build, asset):
     """Section by section, every option the forward path reads has the same value in the generated model and in
     the shipped asset (text level, with the reference's own line grammar)."""
     gen = cfgs.parse_text(cfgs.to_text(build()))
-    ref = cfgs.parse_text(open(os.path.join(REF_BIN, asset)).read())
+    ref = util.reference()["cfg_assets"][asset]
     assert len(gen) == len(ref)
     for i, ((tg, og), (tr, orf)) in enumerate(zip(gen, ref)):
         assert tg == tr, (i, tg, tr)
@@ -45,38 +44,40 @@ def test_generated_cfg_text_equals_reference_asset(name, build, asset):
             assert vg == vr, (name, i, tg, k, vg, vr)
 
 
-@pytest.mark.skipif(not (os.path.isdir(REF_BIN) and util.have_ref()), reason="reference tree / oracle build absent")
+def _assert_same_network(a, key):
+    """The product parser's network `a` == the reference parser's recorded view of the same model (tests/golden/
+    reference_arrays.npz, "parse_<key>_*")."""
+    g = {k[len(key) + 7:]: v for k, v in util.reference_arrays().items() if k.startswith(f"parse_{key}_")}
+    n, batch, h, w, c, inputs = g["net"].tolist()
+    assert a.n == n and a.batch == batch, (key, a.n, n, a.batch, batch)
+    assert (a.h, a.w, a.c, a.inputs) == (h, w, c, inputs), key
+    for i, lb in enumerate(g["layers"].tolist()):
+        la = a.layer(i)
+        for k, v in zip(FIELDS, lb):
+            assert la[k] == v, (key, i, k, la[k], v)
+        if la["type_name"] == "YOLO":
+            assert np.array_equal(la["mask"], g[f"l{i}_mask"]), (key, i)
+            assert np.array_equal(la["anchors"], g[f"l{i}_biases"]), (key, i)
+        if la["type_name"] == "REGION":
+            assert np.array_equal(la["anchors"][:2 * la["n"]], g[f"l{i}_biases"]), (key, i)
+        if la["type_name"] == "ROUTE":
+            assert np.array_equal(la["input_layers"], g[f"l{i}_input_layers"]), (key, i)
+    assert np.array_equal(a.input_calibration(), g["input_calibration"]), key
+
+
 @pytest.mark.parametrize("name,build,asset,qs", [(a[0], a[1], a[2], (0, 1) if a[0] in ("tiny", "xnor") else (1,))
                                                  for a in ASSETS if a[0] in ("tiny", "xnor", "yolov3")])
 def test_generated_cfg_equals_reference_asset(name, build, asset, qs, workdir):
-    """...and the reference's own parser builds identical networks from both files."""
-    from oracle import ref
+    """...and the generated file builds the network the reference's own parser builds from the shipped asset."""
+    import yolo2_light_b200 as yb
     p = cfgs.write_cfg(build(), os.path.join(workdir, "gen_" + name + ".cfg"))
     for q in qs:
-        a = ref.RefNet(p, None, 1, q, 0)
-        b = ref.RefNet(os.path.join(REF_BIN, asset), None, 1, q, 0)
-        assert a.n == b.n
-        for i in range(a.n):
-            la, lb = a.layers[i], b.layers[i]
-            for k in la:
-                if k != "bflops":
-                    assert la[k] == lb[k], (name, i, k, la[k], lb[k])
-            if la["type_name"] in ("YOLO", "REGION"):
-                na = 2 * (la["total"] if la["type_name"] == "YOLO" else la["n"])
-                assert np.array_equal(a.array(i, "biases", na), b.array(i, "biases", na))
-            if la["type_name"] == "YOLO":
-                assert np.array_equal(a.array(i, "mask", la["n"], np.int32), b.array(i, "mask", la["n"], np.int32))
-            if la["type_name"] == "ROUTE":
-                assert np.array_equal(a.array(i, "input_layers", la["n"], np.int32),
-                                      b.array(i, "input_layers", la["n"], np.int32))
-        assert np.array_equal(a.input_calibration(), b.input_calibration())
+        _assert_same_network(yb.parse_network_cfg(p, 1, q), f"{asset}_q{q}")
 
 
-@pytest.mark.skipif(not util.have_ref(), reason="oracle/_ref not built")
 @pytest.mark.parametrize("name", list(util.ZOO) + ["full_tiny", "full_xnor"])
 def test_product_parser_equals_reference_parser(name, workdir):
     import yolo2_light_b200 as yb
-    from oracle import ref
     if name.startswith("full_"):
         secs = cfgs.yolov3_tiny() if name == "full_tiny" else cfgs.tiny_yolo_obj_xnor()
         cfg = cfgs.write_cfg(secs, os.path.join(workdir, name + ".cfg"))
@@ -84,21 +85,8 @@ def test_product_parser_equals_reference_parser(name, workdir):
         cfg, _ = util.model_files(name, workdir)
     for q in (0, 1):
         a = yb.parse_network_cfg(cfg, 3, q)
-        b = ref.RefNet(cfg, None, 3, q, 0)
-        assert a.n == b.n and a.batch == b.batch == 3
-        assert (a.h, a.w, a.c, a.inputs) == (b.height, b.width, b.channels, b.inputs)
-        for i in range(a.n):
-            la, lb = a.layer(i), b.layers[i]
-            for k in FIELDS:
-                assert la[k] == lb[k], (name, q, i, k, la[k], lb[k])
-            if lb["type_name"] == "YOLO":
-                assert np.array_equal(la["mask"], b.array(i, "mask", lb["n"], np.int32))
-                assert np.array_equal(la["anchors"], b.array(i, "biases", 2 * lb["total"]))
-            if lb["type_name"] == "REGION":
-                assert np.array_equal(la["anchors"][:2 * lb["n"]], b.array(i, "biases", 2 * lb["n"]))
-            if lb["type_name"] == "ROUTE":
-                assert np.array_equal(la["input_layers"], b.array(i, "input_layers", lb["n"], np.int32))
-        assert np.array_equal(a.input_calibration(), b.input_calibration())
+        assert a.batch == 3
+        _assert_same_network(a, f"{name}_q{q}")
 
 
 def test_shape_tracer_agrees_with_product_parser(workdir):

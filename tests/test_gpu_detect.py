@@ -1,6 +1,7 @@
 """Device-side detection decode + NMS of the whole batch (yb_network_detect, SURVEY 8f row 1) against
 (a) the host restatement yb_get_network_boxes, image by image, on the very tensors the device produced, and
-(b) the unmodified reference's get_network_boxes + do_nms_sort (oracle/_ref) run on each image separately."""
+(b) the unmodified reference's get_network_boxes + do_nms_sort run on each image separately (its rows are stored in
+tests/golden/reference_arrays.npz, "detect_*")."""
 import os
 
 import numpy as np
@@ -93,13 +94,14 @@ def test_device_detect_cap_and_empty(workdir):
         net.detect(640, 480, 0.5, 0.45, max_rows=0)
 
 
-@pytest.mark.skipif(not util.have_ref(), reason="reference build absent")
-@pytest.mark.parametrize("name,q", [("tiny", 0), ("tiny", 1), ("xnor", 0)])
+REF_CASES = [("tiny", 0), ("tiny", 1), ("xnor", 0)]
+
+
+@pytest.mark.parametrize("name,q", REF_CASES)
 def test_device_detect_vs_reference_boxes(name, q, workdir):
     """Each image through the unmodified reference (batch 1: its decoder reads item 0 only) vs the batched device path
     in exact (FP32 / INT8 / XNOR) precision."""
     import yolo2_light_b200 as yb
-    from oracle import ref
     B = 3
     cfg, wts = _bigger(name, workdir, 160, 160)
     x = cfgs.synthetic_images(B, 3, 160, 160, seed=45)
@@ -108,10 +110,8 @@ def test_device_detect_vs_reference_boxes(name, q, workdir):
     net.predict(x, quantized=bool(q))
     thresh = 0.2 if name == "tiny" else 0.05
     dets, counts = net.detect(640, 480, thresh, 0.45, max_rows=4096, quantized=bool(q))
-    rnet = ref.RefNet(cfg, wts, 1, q, 7)
     for b in range(B):
-        rnet.predict(x[b:b + 1])
-        theirs = np.delete(rnet.get_boxes(640, 480, thresh, 0.45), 5, axis=1)
+        theirs = util.reference_arrays()[f"detect_{name}_q{q}_b{b}"]
         # forward outputs differ in the last bits (f32 sum order): candidates sitting exactly at the threshold may flip
         assert abs(int(counts[b]) - theirs.shape[0]) <= max(1, theirs.shape[0] // 100), (b, counts[b], theirs.shape)
         if counts[b] == theirs.shape[0] and theirs.shape[0]:

@@ -1,5 +1,5 @@
-"""Parity of the CUDA engine (through the C ABI) against the CPU oracle, the reference build (oracle/_ref) and the
-golden vectors.  GPU box only:  python -m pytest tests -m gpu
+"""Parity of the CUDA engine (through the C ABI) against the CPU oracle, the reference build (oracle/_ref), and the
+golden vectors made by the reference (tests/golden).  GPU box only:  python -m pytest tests -m gpu
 
 Bars (BASELINE.json north_star): XNOR popcounts and INT8 s32 accumulators bit-exact; the float epilogues of
 those paths bit-exact too (same op order as the reference); FP32-variant convolutions: f32 CUDA-core path
@@ -185,16 +185,21 @@ def test_detection_outputs_vs_reference_golden(name, q, workdir):
 
 
 # ---- the drop-in path behind the reference's own loader -----------------------------------------------------
-@pytest.mark.skipif(not util.have_ref(), reason="oracle/_ref not built")
-@pytest.mark.parametrize("name,q", [("tiny64", 0), ("tiny64", 1), ("xnor64", 0)])
+DROPIN_CASES = [("tiny64", 0), ("tiny64", 1), ("xnor64", 0)]
+
+
+@pytest.mark.parametrize("name,q", DROPIN_CASES)
 def test_dropin_from_reference_prepared_layers(name, q, workdir):
-    """Model parsed, loaded, folded, binarised and quantised by the REFERENCE's host code; its arrays handed to the
-    engine as yb_layer_desc[] (what INTEGRATION.md's glue does); result vs the reference's own predict."""
+    """Model parsed, loaded, folded, binarised and quantised the way the REFERENCE's host code does it (arrays bit-identical
+    to its own, checked against their digests); those arrays handed to the engine as yb_layer_desc[] (what INTEGRATION.md's
+    glue does); result vs the reference's own predict and decoder (tests/golden)."""
     import ctypes as C
     import yolo2_light_b200 as yb
-    from oracle import ref
+    from test_host_prep import assert_prepared_like_reference
     cfg, wts = util.model_files(name, workdir)
-    rnet = ref.RefNet(cfg, wts, 1, q, 7)
+    prepared = yb.load_network(cfg, wts, batch=1, quantized=q)
+    layers = prepared.layers
+    assert_prepared_like_reference(layers, name, q)
     keep, descs = [], []
 
     def ptr(arr, ctype):
@@ -203,7 +208,7 @@ def test_dropin_from_reference_prepared_layers(name, q, workdir):
         keep.append(arr)
         return arr.ctypes.data_as(C.POINTER(ctype))
 
-    for i, L in enumerate(rnet.layers):
+    for i, L in enumerate(layers):
         d = yb.LayerDesc()
         for k in ("type", "activation", "batch_normalize", "h", "w", "c", "n", "size", "stride", "pad", "out_h",
                   "out_w", "out_c", "xnor", "quantized", "index", "classes", "coords", "softmax", "total", "reverse"):
@@ -211,34 +216,33 @@ def test_dropin_from_reference_prepared_layers(name, q, workdir):
         d.scale = L["scale"]
         t = L["type_name"]
         if t == "CONVOLUTIONAL":
-            nw = L["n"] * L["c"] * L["size"] ** 2
-            d.weights = ptr(rnet.array(i, "weights", nw), C.c_float)
-            d.biases = ptr(rnet.array(i, "biases", L["n"]), C.c_float)
+            d.weights = ptr(np.ascontiguousarray(L["weights"], np.float32), C.c_float)
+            d.biases = ptr(np.ascontiguousarray(L["biases"], np.float32), C.c_float)
             if q:
-                d.weights_int8 = ptr(rnet.array(i, "weights_int8", nw, np.int8), C.c_int8)
+                d.weights_int8 = ptr(np.ascontiguousarray(L["weights_int8"], np.int8), C.c_int8)
                 d.weights_quant_multipler = L["weights_quant_multipler"]
                 d.input_quant_multipler = L["input_quant_multipler"]
             if L["xnor"]:
-                d.mean_arr = ptr(rnet.array(i, "mean_arr", L["n"]), C.c_float)
+                d.mean_arr = ptr(np.ascontiguousarray(L["mean_arr"], np.float32), C.c_float)
         elif t == "ROUTE":
-            d.input_layers = ptr(rnet.array(i, "input_layers", L["n"], np.int32), C.c_int)
+            d.input_layers = ptr(np.ascontiguousarray(L["input_layers"], np.int32), C.c_int)
         elif t == "YOLO":
-            d.mask = ptr(rnet.array(i, "mask", L["n"], np.int32), C.c_int)
-            d.anchors = ptr(rnet.array(i, "biases", 2 * L["total"]), C.c_float)
+            d.mask = ptr(np.ascontiguousarray(L["mask"], np.int32), C.c_int)
+            d.anchors = ptr(np.ascontiguousarray(L["anchors"], np.float32), C.c_float)
         elif t == "REGION":
-            d.anchors = ptr(rnet.array(i, "biases", 2 * L["n"]), C.c_float)
+            d.anchors = ptr(np.ascontiguousarray(L["anchors"], np.float32), C.c_float)
         descs.append(d)
-    net = yb.network_from_layers(descs, 1, rnet.height, rnet.width, rnet.channels, q)
+    net = yb.network_from_layers(descs, 1, prepared.h, prepared.w, prepared.c, q)
     net.set_precision(yb.YB_PREC_FP32)
     x = util.images(name, 1)
-    rnet.predict(x)
     net.predict(x, quantized=bool(q))
+    g = np.load(os.path.join(util.GOLDEN, f"{name}_q{q}.npz"))          # the reference's predict of this very image
     for i, o in net.detection_outputs().items():
-        r = rnet.output(i)
+        r = g[f"b0_out{i}"]
         assert util.rel_l2(o, r.reshape(o.shape)) <= (2e-3 if q else 1e-5), (name, q, i)
     # decoded boxes agree with the reference's get_network_boxes + do_nms_sort
     mine = net.get_network_boxes(0, 640, 480, 0.3, 0.45)
-    theirs = rnet.get_boxes(640, 480, 0.3, 0.45)
+    theirs = util.reference_arrays()[f"dropin_{name}_q{q}_boxes"]
     assert mine.shape[0] == theirs.shape[0]
     if mine.shape[0]:
         a = mine[np.lexsort(mine[:, :4].T[::-1])]
@@ -327,12 +331,15 @@ def test_device_input_pipeline_bit_exact(src_hw, workdir):
         assert util.bits_equal(o, a[i])
 
 
-@pytest.mark.parametrize("name", ["tiny64", "v3_32"])
+CALIB_NAMES = ["tiny64", "v3_32"]
+
+
+@pytest.mark.parametrize("name", CALIB_NAMES)
 def test_int8_calibration_on_device(name, workdir):
     """SURVEY 8f row 3: |x| histograms of every convolution input on the GPU (exact integers) + the reference's KL
-    search; multipliers against entropy_calibration run by the reference on ITS activations, image by image."""
+    search; multipliers against entropy_calibration run by the reference on ITS activations, image by image
+    (tests/golden/reference.json, "device_calibration")."""
     import yolo2_light_b200 as yb
-    from oracle import ref
     B = 2
     cfg, wts = util.model_files(name, workdir)
     x = util.images(name, B)
@@ -351,13 +358,12 @@ def test_int8_calibration_on_device(name, workdir):
     # (2) whole tool
     mult = net.calibrate(x)
     assert mult.shape == (B, len(convs)) and np.all(mult > 0)
-    rnet = ref.RefNet(cfg, wts, 1, 0, 7)
+    expected = util.reference()["device_calibration"][name]
     same = total = 0
     for b in range(B):
-        rnet.predict(x[b:b + 1])
+        assert len(expected[b]) == len(convs)
         for k, i in enumerate(convs):
-            src = x[b] if i == 0 else rnet.output(i - 1)
-            theirs = ref.entropy_calibration(src)
+            theirs = expected[b][k]
             total += 1
             same += np.float32(theirs) == mult[b, k]
             # activations differ in the last bit (f32 summation order): a count may cross a bin edge and move the optimum
@@ -397,15 +403,18 @@ def test_maxpool_fused_with_quantise_or_binarise_is_bit_exact(name, q, workdir):
 
 
 # ---- XNOR layers outside the bit GEMM's shape (stride != 1 or pad != 1): the reference's float-GEMM fallback ----------
-@pytest.mark.skipif(not util.have_ref(), reason="oracle/_ref not built")
-def test_xnor_stride_pad_fallback_matches_reference(workdir):
-    """yolov2_forward_network.c:40-50 + :204: such layers binarise the input to +-1 floats, swap in +-mean weights and run the
-    ordinary im2col + gemm_nn.  The engine does the same (k_binarize_pm1 + exact-order float conv): bit-identical."""
-    import yolo2_light_b200 as yb
-    from oracle import ref
-    secs = [cfgs._net(32, 32), cfgs._conv(8, 3), cfgs._conv(16, 3, 2, xnor=1), cfgs._conv(16, 1, xnor=1),
+def xnor_fallback_model():
+    return [cfgs._net(32, 32), cfgs._conv(8, 3), cfgs._conv(16, 3, 2, xnor=1), cfgs._conv(16, 1, xnor=1),
             cfgs._conv(16, 3, xnor=1),                      # an ordinary XNOR layer behind them
             cfgs._conv(18, 1, bn=False, act="linear"), cfgs._yolo("0,1,2", cfgs.COCO_ANCHORS, 9, classes=1)]
+
+
+def test_xnor_stride_pad_fallback_matches_reference(workdir):
+    """yolov2_forward_network.c:40-50 + :204: such layers binarise the input to +-1 floats, swap in +-mean weights and run the
+    ordinary im2col + gemm_nn.  The engine does the same (k_binarize_pm1 + exact-order float conv): bit-identical to the
+    reference's outputs (tests/golden/reference.json, "xnor_fallback")."""
+    import yolo2_light_b200 as yb
+    secs = xnor_fallback_model()
     cfg = cfgs.write_cfg(secs, os.path.join(workdir, "xnor_fb.cfg"))
     wts = cfgs.write_weights(secs, os.path.join(workdir, "xnor_fb.weights"), seed=23)
     B = 2
@@ -413,15 +422,14 @@ def test_xnor_stride_pad_fallback_matches_reference(workdir):
     net = yb.load_network(cfg, wts, batch=B)
     net.set_option("fuse", 0)
     net.predict(x)
-    rnet = ref.RefNet(cfg, wts, 1, 0, 7)
     for b in range(B):
-        rnet.predict(x[b:b + 1])
         for i in range(4):
-            got = net.fetch_layer(i)[b]
-            exp = rnet.output(i)[0]
-            assert util.bits_equal(got, exp), (b, i, float(np.abs(got - exp).max()))
-        for i, o in net.detection_outputs().items():
-            assert util.rel_l2(o[b], rnet.output(i)[0].reshape(o[b].shape)) <= 1e-3
+            assert util.digest(net.fetch_layer(i)[b]) == util.reference()["xnor_fallback"][b][i], (b, i)
+        outs = net.detection_outputs()
+        assert list(outs) == [len(secs) - 2]
+        for i, o in outs.items():
+            exp = util.reference_arrays()[f"xnor_fallback_b{b}"]
+            assert util.rel_l2(o[b], exp.reshape(o[b].shape)) <= 1e-3
 
 
 # ---- stem + max-pool + quantise / binarise in one kernel (exact nets) ------------------------------------------------------

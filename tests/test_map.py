@@ -1,6 +1,7 @@
 """mAP accounting (SURVEY 8f row 4): yb_map_evaluate against the reference's validate_detector_map
 (additionally.c:4541-4898) on a small synthetic dataset -- BMP images + label files on disk, the reference's own CPU
-forward and decoder on both sides, so only the bookkeeping under test differs."""
+forward and decoder on both sides, so only the bookkeeping under test differs.  The reference's detections of each image
+and what validate_detector_map printed are stored in tests/golden/reference.json / reference_arrays.npz ("map")."""
 import os
 import re
 
@@ -9,7 +10,7 @@ import pytest
 
 import ybtest_util as util
 
-pytestmark = pytest.mark.skipif(not util.have_ref(), reason="reference build absent")
+MAP_CASES = [("tiny64", 0.5), ("v3_32", 0.5), ("tiny64", 0.75)]
 
 
 def _write_bmp(path, img):   # img: u8 [h, w, 3] RGB
@@ -26,13 +27,9 @@ def _write_bmp(path, img):   # img: u8 [h, w, 3] RGB
     open(path, "wb").write(hdr + dib + bytes(data))
 
 
-@pytest.mark.parametrize("name,iou_thresh", [("tiny64", 0.5), ("v3_32", 0.5), ("tiny64", 0.75)])
-def test_map_accounting_equals_reference(name, iou_thresh, workdir):
-    import yolo2_light_b200 as yb
-    from oracle import ref
-    cfg, wts = util.model_files(name, workdir)
-    rnet = ref.RefNet(cfg, wts, 1, 0, 7)
-    classes = rnet.layers[-1]["classes"]
+def write_mapset(name, iou_thresh, workdir, classes, boxes):
+    """The on-disk validation set: 7 BMP images, labels made from the detections `boxes(k, img)` of image k.  Returns
+    (root, detections per image, truth rows)."""
     root = os.path.join(workdir, f"mapset_{name}_{int(iou_thresh * 100)}")
     os.makedirs(os.path.join(root, "images"), exist_ok=True)
     os.makedirs(os.path.join(root, "labels"), exist_ok=True)
@@ -44,9 +41,7 @@ def test_map_accounting_equals_reference(name, iou_thresh, workdir):
         path = os.path.join(root, "images", f"img{k}.bmp")
         _write_bmp(path, img)
         paths.append(path)
-        x = ref.load_resize_u8(img, rnet.width, rnet.height)[None]      # what load_image + resize_image hand to the net
-        rnet.predict(x)
-        r = np.delete(rnet.get_boxes(1, 1, 0.005, 0.45), 5, axis=1)      # get_network_boxes(net, 1, 1, .005, ...) + NMS
+        r = boxes(k, img)
         rows.append(r)
         # labels: some of the strongest detections (true positives), jittered copies (IoU near the threshold), strays
         lab = []
@@ -71,8 +66,24 @@ def test_map_accounting_equals_reference(name, iou_thresh, workdir):
     open(os.path.join(root, "names.txt"), "w").write("\n".join(f"c{i}" for i in range(classes)) + "\n")
     datacfg = os.path.join(root, "data.cfg")
     open(datacfg, "w").write(f"classes = {classes}\nvalid = {root}/valid.txt\nnames = {root}/names.txt\n")
+    return root, rows, truth
 
-    out = ref.validate_map(datacfg, cfg, wts, 0.24, 0, iou_thresh, os.path.join(root, "ref_stdout.txt"))
+
+def _reference_boxes(k, img, key="tiny64_50"):
+    """The reference's get_network_boxes(net, 1, 1, .005, ...) + NMS on load_image + resize_image of image k."""
+    return util.reference_arrays()[f"map_{key}_img{k}"]
+
+
+@pytest.mark.parametrize("name,iou_thresh", MAP_CASES)
+def test_map_accounting_equals_reference(name, iou_thresh, workdir):
+    import yolo2_light_b200 as yb
+    key = f"{name}_{int(iou_thresh * 100)}"
+    rec = util.reference()["map"][key]
+    classes = rec["classes"]
+    root, rows, truth = write_mapset(name, iou_thresh, workdir, classes, lambda k, img: _reference_boxes(k, img, key))
+    out = rec["stdout"]
+    with open(os.path.join(root, "ref_stdout.txt"), "w") as f:
+        f.write(out)
     ap_ref = {int(m.group(1)): float(m.group(2)) for m in re.finditer(r"class_id = (\d+), name = \S+,\s+ap = ([0-9.]+) %", out)}
     m = re.search(r"(?:mean average precision \(mAP\)|average precision \(AP\)) = ([0-9.]+)", out)
     assert m and len(ap_ref) == classes, out[-400:]
@@ -97,7 +108,6 @@ def test_dataset_reader_matches_what_the_reference_reads(workdir):
     """BMP / PPM decode, the label-path rewriting and the label parser of yolo2_light_b200.dataset on the files the
     mAP parity test writes: the reference's loader must see the same pixels (its resize of them == ours of them)."""
     from yolo2_light_b200 import dataset
-    from oracle import ref
     root = os.path.join(workdir, "reader")
     os.makedirs(os.path.join(root, "images"), exist_ok=True)
     os.makedirs(os.path.join(root, "labels"), exist_ok=True)
@@ -127,18 +137,15 @@ def test_map_driver_loop_equals_reference_end_to_end(workdir):
     """dataset.evaluate_map (the loop of tools/map.py) with the forward + decoder supplied by the reference through a
     stand-in object: same files in, same mAP out as validate_detector_map.  (The GPU stand-ins of the two calls are
     parity-tested on their own: test_gpu_detect.py, test_device_input_pipeline_bit_exact.)"""
-    import yolo2_light_b200 as yb
     from yolo2_light_b200 import dataset
-    from oracle import ref
     name = "tiny64"
-    cfg, wts = util.model_files(name, workdir)
-    rnet = ref.RefNet(cfg, wts, 1, 0, 7)
-    classes = rnet.layers[-1]["classes"]
+    classes = util.reference()["map"]["tiny64_50"]["classes"]
     root = os.path.join(workdir, "mapset_tiny64_50")          # written by test_map_accounting_equals_reference
-    if not os.path.exists(os.path.join(root, "data.cfg")):
+    if not os.path.exists(os.path.join(root, "ref_stdout.txt")):
         test_map_accounting_equals_reference(name, 0.5, workdir)
     paths, names, truth = dataset.load_validation_set(os.path.join(root, "data.cfg"))
     assert len(paths) == 7 and len(names) == classes and truth.shape[0] > 0
+    image_index = {dataset.read_image_u8(p).tobytes(): k for k, p in enumerate(paths)}
 
     class RefBacked:
         batch = 2                                               # exercises the padded last batch (7 images)
@@ -147,10 +154,8 @@ def test_map_driver_loop_equals_reference_end_to_end(workdir):
             self.imgs = imgs
 
         def detect(self, w, h, thresh, nms, relative=1, letter=0, max_rows=1024, quantized=False):
-            dets = []
-            for im in self.imgs:
-                rnet.predict(ref.load_resize_u8(im, rnet.width, rnet.height)[None])
-                dets.append(np.delete(rnet.get_boxes(w, h, thresh, nms), 5, axis=1))
+            assert (w, h, thresh, nms) == (1, 1, 0.005, 0.45)   # the settings the stored detections were made with
+            dets = [_reference_boxes(image_index[im.tobytes()], im) for im in self.imgs]
             return dets, np.array([d.shape[0] for d in dets], np.int32)
 
     mAP, aps, st = dataset.evaluate_map(RefBacked(), paths, truth, classes, 0.5, 0.24)

@@ -1,47 +1,40 @@
-"""Pins the CPU restatement (oracle/yolo_oracle.c) against the UNMODIFIED reference (oracle/_ref/
-libyolo2ref_scalar.so, built from /root/reference by oracle/Makefile): whole networks, every layer, bit-for-bit."""
+"""Pins the CPU restatement (oracle/yolo_oracle.c) against the UNMODIFIED reference: whole networks, every layer,
+bit-for-bit (digests of the reference's outputs in tests/golden/reference.json, "layers" and "resize")."""
 import numpy as np
 import pytest
 
 import ybtest_util as util
 
-pytestmark = pytest.mark.skipif(not util.have_ref(), reason="oracle/_ref/libyolo2ref_scalar.so not built")
+WHOLE_NETWORK_CASES = [("tiny64", 0), ("tiny64", 1), ("xnor64", 0), ("v3_32", 0), ("spp32", 0), ("v2voc32", 0),
+                       ("tinyvoc64", 1), ("v3_32", 1), ("tiny_w96_h64", 0), ("tiny_w96_h64", 1), ("v3_w64_h96", 0)]
+RESIZE_SHAPES = [(480, 640, 608, 608), (37, 53, 64, 96), (64, 64, 64, 64), (1, 7, 32, 32), (100, 1, 32, 32)]
 
 
-def _ref_and_port(name, workdir, quantized, batch=1):
+def _assert_port_equals_reference(name, workdir, quantized, batch=1):
     import yolo2_light_b200 as yb
-    from oracle import port, ref
+    from oracle import port
     cfg, wts = util.model_files(name, workdir)
     x = util.images(name, batch)
-    rnet = ref.RefNet(cfg, wts, batch, quantized, 7)
-    rnet.predict(x)
     net = yb.load_network(cfg, wts, batch=batch, quantized=quantized)
     outs = port.run_network(net.layers, x, quantized=bool(quantized))
-    return rnet, outs
+    rec = util.reference()["layers"][f"{name}_q{quantized}_b{batch}"]
+    assert len(outs) == len(rec)
+    for i, (o, (type_name, shape, dig)) in enumerate(zip(outs, rec)):
+        assert o.size == np.prod(shape), (i, o.shape, shape)
+        assert util.digest(o) == dig, f"{name} q={quantized} layer {i} {type_name}"
 
 
-@pytest.mark.parametrize("name,quantized", [("tiny64", 0), ("tiny64", 1), ("xnor64", 0), ("v3_32", 0),
-                                            ("spp32", 0), ("v2voc32", 0), ("tinyvoc64", 1), ("v3_32", 1),
-                                            ("tiny_w96_h64", 0), ("tiny_w96_h64", 1), ("v3_w64_h96", 0)])
+@pytest.mark.parametrize("name,quantized", WHOLE_NETWORK_CASES)
 def test_whole_network_bit_exact(name, quantized, workdir):
     """Same cfg, same generated .weights, same image -> every layer output of the restatement equals the
     reference's l.output bit-for-bit (FP32 conv: identical k-ascending float accumulation; XNOR / INT8: exact
     integers + identical float epilogue; small layers: copies / compares / libm)."""
-    rnet, outs = _ref_and_port(name, workdir, quantized)
-    for i, o in enumerate(outs):
-        r = rnet.output(i)
-        assert o.size == r.size, (i, o.shape, r.shape)
-        assert util.bits_equal(o.reshape(r.shape), r), (
-            f"{name} q={quantized} layer {i} {rnet.layers[i]['type_name']}: "
-            f"max abs diff {np.abs(o.reshape(r.shape) - r).max()}")
+    _assert_port_equals_reference(name, workdir, quantized)
 
 
 def test_batch_two_fp32(workdir):
     """The reference's FP32/XNOR loops handle l.batch > 1 (yolov2_forward_network.c:111, :212); so does the port."""
-    rnet, outs = _ref_and_port("xnor64", workdir, 0, batch=2)
-    for i, o in enumerate(outs):
-        r = rnet.output(i)
-        assert util.bits_equal(o.reshape(r.shape), r), i
+    _assert_port_equals_reference("xnor64", workdir, 0, batch=2)
 
 
 def test_quantize_input_matches_reference_cast():
@@ -63,10 +56,15 @@ def test_quantize_input_matches_reference_cast():
     assert q.tolist() == exp
 
 
-@pytest.mark.parametrize("shape", [(480, 640, 608, 608), (37, 53, 64, 96), (64, 64, 64, 64), (1, 7, 32, 32), (100, 1, 32, 32)])
+def resize_input(h, w):
+    return np.random.default_rng(h * 1000 + w).integers(0, 256, (h, w, 3), dtype=np.uint8)
+
+
+@pytest.mark.parametrize("shape", RESIZE_SHAPES)
 def test_image_pipeline_port_equals_reference(shape):
     """u8 -> float/255 -> resize_image: the port against the reference's own functions, bit-for-bit."""
-    from oracle import port, ref
+    from oracle import port
     h, w, oh, ow = shape
-    img = np.random.default_rng(h * 1000 + w).integers(0, 256, (h, w, 3), dtype=np.uint8)
-    assert util.bits_equal(port.load_resize_u8(img, ow, oh), ref.load_resize_u8(img, ow, oh))
+    got = port.load_resize_u8(resize_input(h, w), ow, oh)
+    assert got.shape == (3, oh, ow)
+    assert util.digest(got) == util.reference()["resize"][f"{h},{w},{oh},{ow}"]

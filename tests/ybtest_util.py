@@ -1,4 +1,8 @@
-"""Shared helpers for the test-suite: small model zoo (generated cfg + seeded weights), reference/oracle access."""
+"""Shared helpers for the test-suite: small model zoo (generated cfg + seeded weights), the stored results of the
+reference (tests/golden)."""
+import functools
+import hashlib
+import json
 import os
 import sys
 
@@ -43,9 +47,28 @@ def images(name, batch):
     return cfgs.synthetic_images(batch, 3, h, w, seed=iseed)
 
 
-def have_ref():
-    from oracle import ref
-    return ref.available("scalar")
+@functools.lru_cache(maxsize=None)
+def reference():
+    """What the original project's CPU code computed for the tests that compare with it (tests/golden/make_reference_golden.py)."""
+    with open(os.path.join(GOLDEN, "reference.json")) as f:
+        return json.load(f)
+
+
+@functools.lru_cache(maxsize=None)
+def reference_arrays():
+    return dict(np.load(os.path.join(GOLDEN, "reference_arrays.npz")))
+
+
+def digest(a, dtype=np.float32):
+    """The first 64 bits of the sha256 of the values of `a` as `dtype`: a fingerprint of the flattened array's bits."""
+    return hashlib.sha256(np.ascontiguousarray(a, dtype).tobytes()).hexdigest()[:16]
+
+
+def sampled_rel_l2(out, key, b):
+    """rel_l2 of image `b` of `out` [batch, ...] against the stored sample `key` of the reference's tensor."""
+    g = reference_arrays()
+    idx = g[f"{key}_b{b}_idx"]
+    return rel_l2(np.asarray(out[b]).ravel()[idx], g[f"{key}_b{b}_val"])
 
 
 def rel_l2(a, b):
